@@ -1,6 +1,6 @@
 """Headline benchmark: WavLM forward+backward throughput in audio-seconds/second (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--model base|large] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--model base|large] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload = the model BASELINE.json's metric names: WavLM-Large, batch 8 x 20 s synthetic 16 kHz waveform per GPU (configs[2]'s
 per-GPU batch; it fits one B200), masking on, fwd + bwd of the whole encoder through the public API (`WavLM.extract_features` +
@@ -279,8 +279,9 @@ class Workload:
             return self.pretrain_step(wav, e2e, collective)
         self._mark("start")
         nvtx.range_push("forward")
-        x, _ = model.extract_features(wav, padding_mask=self.pad_host, mask=True)
+        x, fpm = model.extract_features(wav, padding_mask=self.pad_host, mask=True)
         loss = (x.float() * self.R).sum()
+        self.outputs = {"hidden": x, "padding_mask": fpm, "loss": loss}
         nvtx.range_pop()
         self._mark("forward")
         sync = self._sync_for(collective)
@@ -307,6 +308,7 @@ class Workload:
         out = model(wav, target_list=self.labels, padding_mask=self.pad_host, mask=True)
         lw = [10.0, 10.0, 0.0, 0.1] if self.sat else [10.0]   # features_pen, loss_spk_m, loss_spk_u, diversity (prob_perplexity)
         loss, sample_size, _ = model.criterion(out, pred_masked_weight=1.0, pred_nomask_weight=0.0, loss_weights=lw)
+        self.outputs = {"hidden": out["x"], "padding_mask": out["padding_mask"], "loss": loss}
         nvtx.range_pop()
         self._mark("forward")
         sync = self._sync_for(collective)
@@ -384,7 +386,7 @@ class Workload:
                 f"{self.cfg.mask_prob}, {drop}, all-False padding mask")
 
     def free(self):
-        self.model = self.R = self.wav_dev = self.opt = self.sync = None
+        self.model = self.R = self.wav_dev = self.opt = self.sync = self.outputs = None
         torch.cuda.empty_cache()
 
 
@@ -476,6 +478,32 @@ def quick_line(w: Workload, steps: int, warmup: int, e2e: bool = True):
     return out
 
 
+DUMP_BYTES = 60 * 10**6   # --dump-outputs: float32 payload in all (the .npy headers keep it well inside 64 MB)
+
+
+def dump_outputs(w: Workload, out_dir: str):
+    """--dump-outputs: what the last step handed its caller, as float32 `<name>.npy` files, so that two builds can be compared
+    output for output: the encoder output (`hidden`), the frame padding mask, the loss, and the gradients of all parameters
+    (`grads`; for the optimisation-step workloads, which consume their gradients, the updated parameters, `params`) concatenated
+    in `parameters()` order, which does not depend on how the engine lays out its buffers.  Smallest first, each array gets an
+    equal share of what is left of DUMP_BYTES; an array larger than its share is replaced by a fixed sample of its flattened
+    elements (positions drawn from a generator seeded with 0, sorted)."""
+    import numpy as np
+    arrays = {k: v for k, v in w.outputs.items() if v is not None}
+    params = [p if w.pretrain else p.grad for p in w.model.parameters()]
+    arrays["params" if w.pretrain else "grads"] = torch.cat([t.detach().reshape(-1).float() for t in params if t is not None])
+    os.makedirs(out_dir, exist_ok=True)
+    left = DUMP_BYTES // 4
+    items = sorted(arrays.items(), key=lambda kv: kv[1].numel())
+    for i, (name, t) in enumerate(items):
+        n = min(t.numel(), left // (len(items) - i))
+        if n < t.numel():
+            pos = torch.randint(t.numel(), (n,), generator=torch.Generator().manual_seed(0)).sort().values
+            t = t.reshape(-1)[pos.to(t.device)]
+        left -= n
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def graph_probe(args):
     """The fixed-length fwd+bwd workload captured as ONE CUDA graph (unispeech_b200.graphed.GraphedForwardBackward): device time per
     replayed step, the same with the batch coming from pinned host memory, and what the HOST spends per step (span-mask sampling +
@@ -543,6 +571,8 @@ def main():
                     "rank 0, mean of 3 extra steps) to the line")
     ap.add_argument("--graph-probe", action="store_true", help="(internal) measure the whole step as one CUDA graph "
                     "(unispeech_b200/graphed.py) and print a small JSON object; the default run calls this in a child process")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed (encoder "
+                    "output, padding mask, loss, a fixed sample of the gradients) as DIR/<name>.npy, float32, under 64 MB")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
@@ -570,6 +600,10 @@ def main():
         dist.init_process_group("nccl", device_id=dev)
     assert world == args.gpus, f"--gpus {args.gpus} but WORLD_SIZE={world}"
 
+    # the span masks are drawn from numpy's global generator (the reference's sampler): seeded, the same arguments give the
+    # same inputs on every run
+    import numpy as np
+    np.random.seed(rank)
     w = Workload(args.model, dev, rank, world, dropout=args.dropout, ragged=args.ragged, pretrain=args.pretrain, sat=args.sat)
     cfg, B, secs, T = w.cfg, w.B, w.secs, w.T
 
@@ -592,6 +626,8 @@ def main():
     ms = w.timed(args.steps, False)
     launches = lc0() - n0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(w, args.dump_outputs)
     for _ in range(2):
         w.step(True)
     ms_e2e = w.timed(args.steps, True)

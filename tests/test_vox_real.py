@@ -1,6 +1,7 @@
 """Real speech, ragged: five utterances of the reference's own sample data (4.4 .. 14.2 s, `tests/golden/vox_real_large2l.npz`, made
 by tools/make_vox_golden.py from the UNMODIFIED reference) as one zero-padded batch with a padding mask, WavLM-Large widths, 2
-layers.  CPU: the oracle against the reference's numbers.  GPU: the kernels against the reference's numbers on the valid frames."""
+layers; the fixture keeps every 12th frame of 16 seeded hidden channels.  CPU: the oracle against the reference's numbers.  GPU:
+the kernels against the reference's numbers on the valid frames."""
 import os
 
 import numpy as np
@@ -32,12 +33,12 @@ def test_oracle_on_real_speech_matches_reference():
     torch.set_num_threads(min(16, os.cpu_count() or 1))
     with torch.no_grad():
         r = O.extract_features(sd, wav, cfg, padding_mask=pmask)
-    rows = torch.from_numpy(g["rows"])
+    rows, cols = torch.from_numpy(g["rows"]), torch.from_numpy(g["cols"])
     fpm = torch.from_numpy(g["frame_padding_mask"])
     assert torch.equal(r["padding_mask"], fpm)
     want = torch.from_numpy(g["x_final"].astype(np.float32))
     keep = ~fpm[:, rows]
-    d = (r["x"][:, rows] - want)[keep].abs()
+    d = (r["x"][:, rows][..., cols] - want)[keep].abs()
     assert d.max().item() < 2e-2 and d.mean().item() < 2e-3, (d.max().item(), d.mean().item())   # fp16 storage of values up to ~20
 
 
@@ -55,12 +56,12 @@ def test_kernels_on_real_speech_match_reference(cuda_device):
                                           output_layer=cfg.encoder_layers)
         xf, _ = m.extract_features(wav.to(cuda_device), padding_mask=pmask)
     torch.cuda.synchronize()
-    rows = torch.from_numpy(g["rows"])
+    rows, cols = torch.from_numpy(g["rows"]), torch.from_numpy(g["cols"])
     pad = torch.from_numpy(g["frame_padding_mask"])
     assert torch.equal(fpm.cpu(), pad)
     keep = ~pad[:, rows]
-    for name, got, want in (("x_final", xf[:, rows.to(xf.device)].float().cpu(), torch.from_numpy(g["x_final"].astype(np.float32))),
-                            ("layer1", lr[1][0][rows.to(xf.device)].float().cpu().transpose(0, 1),
+    for name, got, want in (("x_final", xf[:, rows.to(xf.device)].float().cpu()[..., cols], torch.from_numpy(g["x_final"].astype(np.float32))),
+                            ("layer1", lr[1][0][rows.to(xf.device)].float().cpu()[..., cols].transpose(0, 1),
                              torch.from_numpy(g["layer1"].astype(np.float32)).transpose(0, 1))):
         d = (got - want)[keep].abs()
         scale, mscale = want[keep].abs().max().item(), want[keep].abs().mean().item()

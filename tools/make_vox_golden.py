@@ -1,7 +1,8 @@
 """Real-speech ragged fixture: five utterances of the reference's own sample data
 (/root/reference/downstreams/speaker_verification/vox1_data/*/*.wav, 16 kHz int16, 4.4 .. 14.2 s) through the UNMODIFIED reference
 model (oracle/_ref) as ONE zero-padded batch with a sample-level padding mask -- WavLM-Large widths, 2 layers, deterministic weights.
-The waveforms travel with the fixture (the GPU box has no /root/reference); of the outputs (final hidden state and the first layer's output) every 12th frame is stored, in fp16.
+The waveforms travel with the fixture; of the outputs (final hidden state and the first layer's output) every 12th frame of 16 seeded
+channels is stored, in fp16, which keeps the file under 1 MB.
 
     python -m oracle.build_ref && python tools/make_vox_golden.py        (authoring container only)
 """
@@ -19,6 +20,7 @@ from oracle import build_ref  # noqa: E402
 from oracle import wavlm_oracle as O  # noqa: E402
 
 STEP = 12
+CHANNELS = 16
 PICK = ["Lea_Thompson/mHTAr5dlAgc_0000004.wav", "David_Faustino/hn8GyCJIfLM_0000012.wav", "Zulay_Henao/WbB8m9-wlIQ_0000001.wav",
         "Zulay_Henao/gFfcgOVmiO0_0000002.wav", "Josh_Gad/RFyw7V3SOnQ_0000001.wav"]
 
@@ -45,10 +47,11 @@ def main():
         xf, _ = m.extract_features(wav.clone(), padding_mask=pmask, mask=False)
     T = xf.shape[1]
     rows = np.arange(0, T, STEP)
+    cols = np.sort(np.random.default_rng(0).choice(xf.shape[2], CHANNELS, replace=False))
     out = os.path.join(ROOT, "tests", "golden", "vox_real_large2l.npz")
-    np.savez_compressed(out, pcm=pcm, lengths=np.asarray(lengths), rows=rows, frame_padding_mask=fpm.numpy(),
-                        x_final=xf[:, rows].numpy().astype(np.float16),
-                        layer1=lr[1][0][rows].numpy().astype(np.float16))
+    np.savez_compressed(out, pcm=pcm, lengths=np.asarray(lengths), rows=rows, cols=cols, frame_padding_mask=fpm.numpy(),
+                        x_final=xf[:, rows][..., cols].numpy().astype(np.float16),
+                        layer1=lr[1][0][rows][..., cols].numpy().astype(np.float16))
     print("T", T, "rows", len(rows), "valid frames", (~fpm).sum(1).tolist(), "bytes", os.path.getsize(out))
 
 
