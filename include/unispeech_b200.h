@@ -105,7 +105,8 @@ int b200s_posconv_wgrad(const void* dy, long long dy_bs, long long dy_rs, const 
  * Replaces compute_bias + gate multiply + F.multi_head_attention_forward (WavLM/modules.py:417-455,504-563); the
  * [B*H,T,T] bias is never materialised (it is Toeplitz).  qkv: bf16 [B,T,3D] fused projection output; gate: fp32
  * [B,H,T] or NULL (=1); tab: fp32 [H,2T-1] or NULL (no bias); key_pad: uint8 [B,T] or NULL; out: bf16 [B,T,D];
- * lse: fp32 [B,H,T] log2-domain log-sum-exp (saved for backward).  head_dim = 64, T <= 4096. */
+ * lse: fp32 [B,H,T] log2-domain log-sum-exp (saved for backward).  head_dim = 64; T <= b200s_attn_fwd_max_frames(tab != NULL)
+ * (3072 with the bias, 16384 without): the kernel keeps the CTA's table slice and key mask in shared memory. */
 int b200s_attn_fwd(const void* qkv, const float* gate, const float* tab, const uint8_t* key_pad, void* out,
                    float* lse, int B, int T, int H, float scale, b200s_stream stream);
 
@@ -135,6 +136,26 @@ int b200s_attn_bwd_fused_dropout(const void* qkv, const void* out, const void* d
                                  float* dq_acc, void* dqkv, float* dgate, float* dtab, int B, int T, int H, float scale,
                                  float drop_p, const uint32_t* drop_mask, b200s_stream stream);
 long long b200s_attn_dropout_mask_words(int B, int T, int H);
+
+/* Longest T that b200s_attn_fwd accepts, with (has_bias != 0) or without the relative-position table. */
+int b200s_attn_fwd_max_frames(int has_bias);
+
+/* ============================ long-utterance attention (csrc/attn_long.cu) ============================ */
+
+/* Same inputs, outputs and numerics as b200s_attn_fwd (no dropout) for 1 <= T <= 16384, with shared memory that does not
+ * depend on T.  tab is required.  tab_radius R (0 <= R <= T-1) promises tab[h, delta] = tab[h, +-R] for |delta| >= R (the
+ * WavLM bucketing saturates beyond some distance); R = T-1 is exact for any table.  Key tiles whose every (query, key)
+ * distance lies beyond R on one side use the per-row constant gate * tab[h, +-R] and skip the table.  head_dim = 64. */
+int b200s_attn_fwd_long(const void* qkv, const float* gate, const float* tab, int tab_radius, const uint8_t* key_pad,
+                        void* out, float* lse, int B, int T, int H, float scale, b200s_stream stream);
+
+/* Backward of b200s_attn_fwd_long, same contract as b200s_attn_bwd for 1 <= T <= 16384 (tab = NULL: no bias, tab_radius
+ * ignored).  dgate is written; dtab is += and shared by all layers.  With R < T-1 the gradient of every saturated diagonal
+ * |delta| >= R is summed into dtab at delta = +-R and the entries beyond are left untouched: the bucket scatter
+ * (b200s_relpos_table_bwd) then yields the same embedding gradient, since all those deltas share one bucket per side. */
+int b200s_attn_bwd_long(const void* qkv, const void* out, const void* dout, const float* gate, const float* tab,
+                        int tab_radius, const uint8_t* key_pad, const float* lse, float* delta, void* dqkv, float* dgate,
+                        float* dtab, int B, int T, int H, float scale, b200s_stream stream);
 
 /* SMs the persistent CTA-pair GEMM kernels leave free (0 = none, the default).  Data-parallel runs overlap the NCCL gradient exchange
  * with the backward pass; its CTAs (bounded by NCCL_MAX_CTAS) then find free SMs instead of displacing clusters of a grid that was

@@ -494,6 +494,13 @@ __global__ void __launch_bounds__(256, 1) attn_bwd_dq_kernel(const __grid_consta
 
 int make_qkv_tmap(CUtensorMap* out, const void* qkv, int T, int B, int D3, int box_rows);
 
+// Delta = rowsum(dO * O) for the long-utterance backward (attn_long.cu)
+cudaError_t launch_attn_delta(const void* out, const void* dout, int B, int T, int H, float* delta, cudaStream_t st) {
+  const long long rows = static_cast<long long>(B) * T;
+  return launch_pdl(attn_delta_kernel, dim3(static_cast<unsigned>(ceil_div_ll(rows * 32, 256))), dim3(256), 0, st,
+                    static_cast<const __nv_bfloat16*>(out), static_cast<const __nv_bfloat16*>(dout), B, T, H, delta);
+}
+
 }  // namespace b200
 
 using namespace b200;

@@ -72,6 +72,12 @@ constexpr float kRebase = 1.2089258e24f;   // 2^80: a tile whose row sum reaches
 // floats of ONE bias-table copy: (N + 2) * 128 entries + 8 so that consecutive copies start 8 banks apart (conflict-free
 // 128-bit loads across the quarter warp, whose lanes alternate between the four copies)
 __host__ __device__ constexpr int fwd_tab_stride(int N) { return (N + 2) * kAttnTile + 8; }
+// dynamic shared memory of attn_fwd_kernel for N key tiles: table copies (with the bias), key mask, tile flags
+constexpr int fwd_smem_bytes(int N, bool has_bias) {
+  return kFwdTab + static_cast<int>(sizeof(float)) * ((has_bias ? kTabCopies * fwd_tab_stride(N) : 0) + N * kAttnTile) +
+         static_cast<int>(sizeof(int)) * N + 1024;
+}
+constexpr int kFwdSmemMax = 232448 - 1024;
 
 template <bool HAS_BIAS, bool DROP>
 __global__ void __launch_bounds__(kFwdThreads, 1) attn_fwd_kernel(const __grid_constant__ CUtensorMap tm,
@@ -470,9 +476,8 @@ int b200s_attn_fwd_dropout(const void* qkv, const float* gate, const float* tab,
   memset(&p, 0, sizeof(p));
   p.T = T; p.H = H; p.B = B; p.D = D;
   p.n_tiles = ceil_div(T, kAttnTile);
-  const int smem = kFwdTab + sizeof(float) * ((tab != nullptr ? kTabCopies * fwd_tab_stride(p.n_tiles) : 0) + p.n_tiles * kAttnTile) +
-                   sizeof(int) * p.n_tiles + 1024;
-  B200_CHECK_ARG(T >= 1 && smem <= 232448 - 1024, "attn_fwd: T=%d out of range (needs %d bytes of shared memory)", T, smem);
+  const int smem = fwd_smem_bytes(p.n_tiles, tab != nullptr);
+  B200_CHECK_ARG(T >= 1 && smem <= kFwdSmemMax, "attn_fwd: T=%d out of range (needs %d bytes of shared memory)", T, smem);
   if (make_qkv_tmap(&tm, qkv, T, B, 3 * D, kAttnTile)) return -3;
   p.scale = scale;
   p.gate = gate; p.tab = tab; p.key_pad = key_pad;
@@ -500,5 +505,11 @@ int b200s_attn_fwd(const void* qkv, const float* gate, const float* tab, const u
 }
 
 long long b200s_attn_dropout_mask_words(int B, int T, int H) { return attn_drop_mask_words(B, H, T); }
+
+int b200s_attn_fwd_max_frames(int has_bias) {
+  int n = 1;
+  while (fwd_smem_bytes(n + 1, has_bias != 0) <= kFwdSmemMax) ++n;
+  return n * kAttnTile;
+}
 
 }  // extern "C"

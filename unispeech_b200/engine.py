@@ -54,6 +54,38 @@ def relative_positions_bucket_lut(T: int, num_buckets: int, max_distance: int) -
     return (buckets + torch.where(is_small, rp, large)).to(torch.int32)
 
 
+def bias_radius(lut: torch.Tensor, num_buckets: int) -> int:
+    """Smallest r such that every |delta| >= r falls in the last bucket of its side (num_buckets - 1 for delta > 0,
+    num_buckets // 2 - 1 for delta < 0): the log branch of the bucketing clamps there, so tab[h, delta] = tab[h, +-r] beyond.
+    T - 1 when a side never saturates within the utterance.  `lut`: bucket(delta) for delta in [-(T-1), T-1]."""
+    T = (lut.numel() + 1) // 2
+    lut = lut.cpu()
+    nb = num_buckets // 2
+    r = 0
+    for side, last in ((lut[T - 1:], 2 * nb - 1), (lut[:T].flip(0), nb - 1)):   # index = |delta|
+        off = (side != last).nonzero()
+        if off.numel():
+            r = max(r, int(off[-1]) + 1)
+    return min(r, T - 1)
+
+
+ATTN_MAX_FRAMES = 16384   # longest input of the long-utterance attention kernels (csrc/attn_long.cu)
+_T_BWD_FUSED = 2048       # longest input of the fused attention backward (its shared-memory tables grow with T)
+_T_BWD_SPLIT = 4096       # longest input of the two-kernel attention backward (same reason)
+
+
+def attn_kernels(T: int, has_bias: bool):
+    """(forward, backward) attention kernels for T frames.  Shapes the per-CTA-table kernels accept stay on them: forward
+    `attn_fwd` up to its shared-memory limit (3072 frames with the bias, 16384 without), backward the fused kernel up to 2048
+    and `attn_bwd` up to 4096.  Longer inputs, up to ATTN_MAX_FRAMES, run the long-utterance kernels, whose shared memory
+    does not depend on T."""
+    if not 1 <= T <= ATTN_MAX_FRAMES:
+        raise ValueError(f"attention supports 1..{ATTN_MAX_FRAMES} frames (got T={T}, {T / 50:.1f} s of audio)")
+    fwd = "attn_fwd" if T <= ops.attn_fwd_max_frames(has_bias) else "attn_fwd_long"
+    bwd = "attn_bwd_fused" if T <= _T_BWD_FUSED else ("attn_bwd" if T <= _T_BWD_SPLIT else "attn_bwd_long")
+    return fwd, bwd
+
+
 class FlatGrads:
     """One flat fp32 gradient buffer; every parameter's `.grad` is a view into it."""
 
@@ -176,6 +208,7 @@ class Engine:
         self.dev = None
         self.prepared_version = None
         self.lut_cache: Dict[int, torch.Tensor] = {}
+        self.radius_cache: Dict[int, int] = {}
         self.flat: Optional[FlatGrads] = None
         self._params = None
         self.drop: Optional[DR.DropState] = None  # set per forward pass by WavLM._begin (training-mode dropout)
@@ -279,6 +312,12 @@ class Engine:
         if T not in self.lut_cache:
             self.lut_cache[T] = relative_positions_bucket_lut(T, self.cfg.num_buckets, self.cfg.max_distance).to(self.dev)
         return self.lut_cache[T]
+
+    def tab_radius(self, T: int) -> int:
+        """Saturation radius of the bias table for T frames (bias_radius of the cached LUT), for the long attention kernels."""
+        if T not in self.radius_cache:
+            self.radius_cache[T] = bias_radius(self.lut(T), self.cfg.num_buckets)
+        return self.radius_cache[T]
 
     def active_drop(self) -> Optional[DR.DropState]:
         """Dropout state of the current forward pass (None in eval mode or when every probability is 0)."""
@@ -619,10 +658,10 @@ class Engine:
         p_h = d.p if d is not None else 0.0
         p_a = d.p_attn if d is not None else 0.0
         p_act = d.p_act if d is not None else 0.0
-        t_fused = 2048   # longest input of the fused attention backward (its shared-memory tables grow with T)
-        if p_a > 0 and T > t_fused:
-            raise NotImplementedError(f"attention_dropout > 0 is implemented in the fused attention kernels for T <= {t_fused} frames "
-                                      f"(got T={T}); set attention_dropout=0 for longer inputs")
+        if p_a > 0 and T > _T_BWD_FUSED:
+            raise NotImplementedError(f"attention_dropout > 0 is implemented in the fused attention kernels for T <= {_T_BWD_FUSED} "
+                                      f"frames (got T={T}); set attention_dropout=0 for longer inputs")
+        attn_fwd_kernel = attn_kernels(T, tab is not None)[0]
         st = dict(x=x, drop=d)
         rag = self.ragged_valid if pad_u8 is not None else None   # int32 [B] valid frames (ragged batch) or None
         want_gate = tab is not None and cfg.gru_rel_pos
@@ -649,8 +688,10 @@ class Engine:
             dmask = torch.empty(ops.attn_dropout_mask_words(B, T, H), dtype=torch.int32, device=dev)
             ops.attn_fwd_dropout(qkv, gate, tab, pad_u8, ao, lse, B, T, H, 64 ** -0.5, p_a,
                                  d.key(DR.layer_site(idx, DR.L_ATTENTION)), dmask)
-        else:
+        elif attn_fwd_kernel == "attn_fwd":
             ops.attn_fwd(qkv, gate, tab, pad_u8, ao, lse, B, T, H, 64 ** -0.5)
+        else:
+            ops.attn_fwd_long(qkv, gate, tab, self.tab_radius(T), pad_u8, ao, lse, B, T, H, 64 ** -0.5)
         y1 = e(B, T, D)
         if p_h > 0:  # x + dropout1(out_proj(attn)), WavLM/WavLM.py:702-703,726-727
             self._mm(ao, D, w["o"], D, y1, rag, T, B, bias=a.out_proj.bias)
@@ -771,7 +812,8 @@ class Engine:
         delta = f(B, H, T)
         gate = st["gate"]
         dgate = f(B, H, T) if tab is not None else None
-        if T <= 2048:
+        attn_bwd_kernel = attn_kernels(T, tab is not None)[1]
+        if attn_bwd_kernel == "attn_bwd_fused":
             key = (B, T, D)
             if getattr(self, "_dq_acc_key", None) != key:  # fp32 dQ accumulator: zero on entry, re-zeroed by the kernel
                 self._dq_acc = torch.zeros(B, T, D, dtype=torch.float32, device=dev)
@@ -782,9 +824,12 @@ class Engine:
             else:
                 ops.attn_bwd_fused(st["qkv"], st["ao"], dao, gate, tab, pad, st["lse"], delta, self._dq_acc, dqkv, dgate,
                                    dtab if tab is not None else None, B, T, H, 64 ** -0.5)
-        else:
+        elif attn_bwd_kernel == "attn_bwd":
             ops.attn_bwd(st["qkv"], st["ao"], dao, gate, tab, pad, st["lse"], delta, dqkv, dgate,
                          dtab if tab is not None else None, B, T, H, 64 ** -0.5)
+        else:  # (with R < T-1 the saturated diagonals' gradient lands at delta = +-R: same bucket, same embedding gradient)
+            ops.attn_bwd_long(st["qkv"], st["ao"], dao, gate, tab, self.tab_radius(T) if tab is not None else 0, pad, st["lse"],
+                              delta, dqkv, dgate, dtab if tab is not None else None, B, T, H, 64 ** -0.5)
         ops.colsum(dqkv, T * 3 * D, 3 * D, T, B, 3 * D, g(a.q_proj.bias).view(-1), valid=rag)  # q,k,v bias grads are adjacent in the flat buffer
         attn_in = st["xn"] if pre_ln else x
         dxg = None

@@ -256,6 +256,22 @@ def attn_bwd_fused(qkv, out, dout, gate, tab, key_pad, lse, delta, dq_acc, dqkv,
           flops=10.0 * B * H * T * T * 64)
 
 
+def attn_fwd_max_frames(has_bias: bool) -> int:
+    """Longest T `attn_fwd` accepts (its shared-memory footprint grows with T)."""
+    return int(L.load().b200s_attn_fwd_max_frames(int(bool(has_bias))))
+
+
+def attn_fwd_long(qkv, gate, tab, tab_radius, key_pad, out, lse, B, T, H, scale):
+    _call("b200s_attn_fwd_long", L.ptr(qkv), L.ptr(gate), L.ptr(tab), i32(tab_radius), L.ptr(key_pad), L.ptr(out), L.ptr(lse),
+          i32(B), i32(T), i32(H), f32(scale), _s(), flops=4.0 * B * H * T * T * 64)
+
+
+def attn_bwd_long(qkv, out, dout, gate, tab, tab_radius, key_pad, lse, delta, dqkv, dgate, dtab, B, T, H, scale):
+    _call("b200s_attn_bwd_long", L.ptr(qkv), L.ptr(out), L.ptr(dout), L.ptr(gate), L.ptr(tab), i32(tab_radius), L.ptr(key_pad),
+          L.ptr(lse), L.ptr(delta), L.ptr(dqkv), L.ptr(dgate), L.ptr(dtab), i32(B), i32(T), i32(H), f32(scale), _s(),
+          flops=10.0 * B * H * T * T * 64)
+
+
 # ------------------------------------------------------------------------------------------------- dropout
 def u32(v) -> int:
     return int(v) & 0xFFFFFFFF
